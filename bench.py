@@ -40,7 +40,9 @@ RES = 0.02
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=400)   # >= 0.2 s of timed device work at 8192^2
+    # default: 400 (>= 0.2 s of timed device work at 8192^2); 20 for --impl reference and 5 for --workload plugin_chain,
+    # whose steps take seconds (host CPU) and hundreds of milliseconds (host GridMaps, timed twice) each
+    ap.add_argument("--steps", type=int, default=None)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="chain8192", choices=["chain8192", "chain2048", "batched512", "footprint4096", "footprint4096_offset0", "footprint_polygon4096", "slope8192", "plugin_chain"])
@@ -53,7 +55,64 @@ def parse():
     ap.add_argument("--cols", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the layers the last timed step computed as DIR/<name>.npy, their NaN "
+                         "cells as DIR/<name>_nan.npy (see dump_outputs), so that two builds can be compared output for output; "
+                         "--impl reference writes DIR/reference_<name>.npy for its top-left crop, comparable only with itself")
+    args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.impl == "reference" else 5 if args.workload == "plugin_chain" else 400
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload == "plugin_chain":
+        ap.error("--dump-outputs is not available for --workload plugin_chain: its timed passes run inside the C++ harness")
+    return args
+
+
+DUMP_BYTES = 60_000_000  # all .npy files of one --dump-outputs run together stay below 64 MB
+DUMP_SEED = 7
+
+
+def dump_outputs(path, arrays, dist=None, world=1, rank=0):
+    """`--dump-outputs DIR`: write every array of `arrays` (name -> this rank's tensor or column-major numpy layer, all of one
+    size) as DIR/<name>.npy, 1-D in the array's dtype.  The whole array is the ranks' shares concatenated in rank order and
+    flattened in storage order (a column-major layer: index col * rows + row; a batch of maps: one map after the other), so
+    that a run on N GPUs writes the same files as a run on one.  Arrays too large for their share of DUMP_BYTES are written
+    at a sorted, seeded sample of flat indices, which depends only on the size: the same cells in every run and every build.
+    Every written value is finite: a cell where a layer holds NaN (no data; the chain answers so for most cells whose input
+    elevation is NaN) is written as 0.0 in <name>.npy and as 1.0 in DIR/<name>_nan.npy, which holds 0.0 at every other cell,
+    so the two files carry the layer's values and its NaN pattern at every sampled cell.  Collective at N > 1 (every rank
+    calls it); rank 0 writes."""
+    import torch
+
+    def flat(a):
+        return a.reshape(-1) if torch.is_tensor(a) else torch.from_numpy(np.ravel(a, order="F"))
+
+    arrays = {name: flat(a) for name, a in arrays.items()}
+    first = next(iter(arrays.values()))
+    dev, n_local = first.device, first.numel()
+    assert all(a.numel() == n_local for a in arrays.values())
+    n_total = n_local * world
+    k = DUMP_BYTES // (2 * len(arrays)) // max(a.element_size() for a in arrays.values())   # values + NaN pattern
+    if n_total <= k:
+        idx = torch.arange(n_total, device=dev)
+    else:
+        idx = torch.from_numpy(np.unique(np.random.default_rng(DUMP_SEED).integers(0, n_total, k))).to(dev)
+    owner = idx // n_local
+    mine = owner == rank
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        vals = torch.zeros((idx.numel(),), dtype=a.dtype, device=dev)
+        vals[mine] = a.to(dev)[idx[mine] - rank * n_local]
+        if world > 1:
+            parts = [torch.empty_like(vals) for _ in range(world)]
+            dist.all_gather(parts, vals)
+            vals = torch.stack(parts)[owner, torch.arange(idx.numel(), device=dev)]
+        if rank == 0:
+            nan = torch.isnan(vals)
+            np.save(os.path.join(path, name + ".npy"), torch.where(nan, torch.zeros_like(vals), vals).cpu().numpy())
+            np.save(os.path.join(path, name + "_nan.npy"), nan.to(vals.dtype).cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -226,16 +285,18 @@ def run_reference(args):
     g = ob.Geometry.make(n, n, RES)
     p = ob.ChainParams.yaml_defaults(0)
     threads = len(os.sched_getaffinity(0))  # all host threads, also under torchrun (which exports OMP_NUM_THREADS=1)
-    # each step is one pass over the bounded sample; the step count is capped so the whole run ends within minutes
-    steps, warmup = min(args.steps, 20), min(args.warmup, 2)
+    # each step is one pass over the bounded sample; at most two warm-up passes, each takes seconds
+    warmup = min(args.warmup, 2)
     for _ in range(warmup):
         ob.chain(g, p, z, nthreads=threads)
     t0 = time.perf_counter()
-    for _ in range(steps):
-        ob.chain(g, p, z, nthreads=threads)
+    for _ in range(args.steps):
+        o = ob.chain(g, p, z, nthreads=threads)
     dt = time.perf_counter() - t0
-    val = n * n * steps / dt / 1e6
-    args.steps, args.warmup = steps, warmup
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"reference_" + name: layer for name, layer in o.items()})
+    val = n * n * args.steps / dt / 1e6
+    args.warmup = warmup
     out = {"impl": "reference", "metric": "Mcells/s full filter chain, synthetic elevation", "value": val, "unit": "Mcells/s",
            "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
            "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None, "dtype": "f64 compute / f32 layers",
@@ -266,7 +327,7 @@ def run_plugin_chain(args, torch, dev):
     with tempfile.TemporaryDirectory() as tmp:
         src = os.path.join(tmp, "elev.bin")
         z.cpu().numpy().tofile(src)
-        passes = max(2, min(args.steps, 5))
+        passes = args.steps
         for name, fuse in (("fused_registry", "1"), ("standalone_literal", "0")):
             env = dict(os.environ, TE_B200_FUSE_CHAIN=fuse)
             r = subprocess.run([os.path.join(plugin, "test_plugins"), "bench", str(rows), str(cols), repr(RES), src, str(passes)],
@@ -305,6 +366,7 @@ def run_other(args, torch, dist, te, world, rank, local, dev):
         outs = [torch.empty((n, cols, rows), dtype=torch.float32, device=dev) for _ in range(4)]
         cells = n_total * rows * cols
         name = f"{n_total} independent {rows}x{cols} maps, full fused chain, {n} maps per GPU"
+        outputs = dict(zip(("slope", "step", "roughness", "traversability"), outs))
 
         def step():
             ctx.chain_batched(g, prm, n, z, *outs, te.MEM_DEVICE)
@@ -316,6 +378,7 @@ def run_other(args, torch, dist, te, world, rank, local, dev):
         out = torch.empty_like(nz)
         cells = rows * cols
         name = f"SlopeFilter only (te_slope) over a {rows}x{cols} surface_normal_z layer, 8 B/cell"
+        outputs = {"slope": out}
 
         def step():
             ctx.slope(g, 1.0, nz, out, te.MEM_DEVICE)
@@ -332,6 +395,7 @@ def run_other(args, torch, dist, te, world, rank, local, dev):
         out = torch.empty((cols, rows), dtype=torch.float32, device=dev)
         cells = rows * cols
         name = f"footprint sweep r=0.30 m offset={fp.offset:.2f} m over {rows}x{cols} traversability/slope/step/elevation"
+        outputs = {"traversability_footprint": out}
 
         def step():
             ctx.footprint(g, fp, lay[3], lay[0], lay[1], z, out, te.MEM_DEVICE)
@@ -340,6 +404,7 @@ def run_other(args, torch, dist, te, world, rank, local, dev):
             poly = [[0.45, 0.30], [0.45, -0.30], [-0.45, -0.30], [-0.45, 0.30]]
             out2 = torch.empty((cols, rows), dtype=torch.float32, device=dev)
             name = f"polygon footprint sweep (0.9 m x 0.6 m, yaw 0.7854: traversability_x + traversability_rot) over {rows}x{cols}"
+            outputs = {"traversability_x": out, "traversability_rot": out2}
 
             def step():  # noqa: F811
                 ctx.footprint_polygon(g, fp, poly, 0.7854, lay[3], lay[0], lay[1], z, out, out2, te.MEM_DEVICE)
@@ -359,6 +424,8 @@ def run_other(args, torch, dist, te, world, rank, local, dev):
         step()
     ev1.record(stream)
     barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs, dist, world, rank)
     ms = torch.tensor([ev0.elapsed_time(ev1)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -532,6 +599,9 @@ def main():
     ms_total = ev0.elapsed_time(ev1)
     halo_ms = (sum(a.elapsed_time(b) for a, b in hev[:timed[1]]) / max(timed[1], 1)) if world > 1 else 0.0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        last = outsets[(rot[0] - 1) % nsets]
+        dump_outputs(args.dump_outputs, dict(zip(("slope", "step", "roughness", "traversability"), last)), dist, world, rank)
     launches1, slow_cells = ctx.stats()
     # kernel split (fused stencil / fix-up tiers): CUDA events recorded inside the C ABI around the launches, in a SEPARATE short
     # run of the same step — events between the kernels would serialise the programmatic dependent launches of the timed region

@@ -5,7 +5,7 @@ Needs a calibration build, which is the only one that reads TE_FUSED_ROUGH_K / T
     TE_B200_LIBRARY=$PWD/traversability_estimation_b200/libte_b200_calib.so python tools/dev_calib.py
 """
 import os, sys, json
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tools'); sys.path.insert(0, '/root/repo/tests')
+_R = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path[:0] = [_R, _R + '/tools', _R + '/tests']
 import numpy as np, synth, torch, bench
 import traversability_estimation_b200 as te
 from oracle import binding as ob

@@ -1,6 +1,6 @@
 """Dev check: run the fused chain twice on the same map and report cells whose bits differ (GPU)."""
-import sys
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tools')
+import os, sys
+_R = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path[:0] = [_R, _R + '/tools']
 import torch, bench
 import traversability_estimation_b200 as te
 rows = cols = int(sys.argv[1]) if len(sys.argv) > 1 else 4096

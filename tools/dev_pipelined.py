@@ -1,6 +1,6 @@
 """Dev check: pipelined host path vs device path, report differing cells (GPU)."""
-import sys
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tools')
+import os, sys
+_R = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path[:0] = [_R, _R + '/tools']
 import torch, bench
 import traversability_estimation_b200 as te
 rows, cols = 2048, 2304

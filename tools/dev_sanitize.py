@@ -1,5 +1,5 @@
-import sys
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tools'); sys.path.insert(0, '/root/repo/tests')
+import os, sys
+_R = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path[:0] = [_R, _R + '/tools', _R + '/tests']
 import numpy as np, synth
 import traversability_estimation_b200 as te
 ctx = te.Context(0)

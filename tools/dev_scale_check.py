@@ -1,6 +1,6 @@
 """One-off: fused vs literal kernel on the bench map itself (8192 x 8192, 1 % holes)."""
-import sys
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tools')
+import os, sys
+_R = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path[:0] = [_R, _R + '/tools']
 import torch, bench
 import traversability_estimation_b200 as te
 rows = cols = 8192

@@ -1,13 +1,18 @@
-"""Extract the reference's golden vector into tests/golden/ (run in the build container only).
+"""Extract the reference's golden vector into tests/golden/.
 
-Source: /root/reference/traversability_estimation/maps/elevation_map.bag — the reference's
-only known-answer material (SURVEY.md Appendix B).  /root/reference does not exist on the
-GPU box, so the decoded layers are committed as a small .npz next to this script's output
-manifest (crc32 per layer, so a reader can re-derive them from the bag and compare).
+Source: the reference's traversability_estimation/maps/elevation_map.bag — its only
+known-answer material (SURVEY.md Appendix B), kept xz-compressed as
+tests/golden/elevation_map.bag.xz; a path to an uncompressed bag may be given instead.
+The decoded layers are committed as a small .npz next to this script's output manifest
+(crc32 per layer, so a reader can re-derive them from the bag and compare).
+
+    python tools/make_golden.py [path/to/elevation_map.bag]
 """
 import json
+import lzma
 import os
 import sys
+import tempfile
 import zlib
 
 import numpy as np
@@ -15,14 +20,20 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from bag import read_gridmap_bag  # noqa: E402
 
-SRC = "/root/reference/traversability_estimation/maps/elevation_map.bag"
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden")
 KEEP = ["elevation", "traversability_slope", "traversability_step", "traversability_roughness",
         "traversability", "traversability_footprint", "slope_footprint", "step_footprint"]
 
 
 def main():
-    m = read_gridmap_bag(SRC)
+    if len(sys.argv) > 1:
+        m = read_gridmap_bag(sys.argv[1])
+    else:
+        with open(os.path.join(OUT, "elevation_map.bag.xz"), "rb") as f, tempfile.TemporaryDirectory() as tmp:
+            bag = os.path.join(tmp, "elevation_map.bag")
+            with open(bag, "wb") as g:
+                g.write(lzma.decompress(f.read()))
+            m = read_gridmap_bag(bag)
     os.makedirs(OUT, exist_ok=True)
     arrays = {k: m.data[k] for k in KEEP}
     np.savez_compressed(os.path.join(OUT, "fixture_gridmap.npz"), **arrays)
